@@ -4,6 +4,8 @@
   python bench.py --gpus N --steps K --warmup W            (our arm)
   python bench.py --impl reference --gpus N --steps K ...  (CPU arm: the oracle port of the
                                                             reference's InMemoryStorage path)
+  python bench.py ... --dump-outputs DIR                   (also write the last timed step's outputs
+                                                            as DIR/<name>.npy, to compare two builds)
 
 A step = one batch (65536 requests per GPU) of `check_rate_limited_and_update`
 (limitador/src/lib.rs:425-464) through the C-ABI.  `value` is measured with the batch
@@ -113,6 +115,22 @@ def counters_examined(lim: np.ndarray, first: np.ndarray, L: int):
     allowed = lim == 0
     k = (first[~allowed] % L).astype(np.int64) + 1  # C2: limit_id = ns*4 + k
     return int(allowed.sum()) * L + int(k.sum()), int(allowed.sum()) * L
+
+
+def dump_outputs(out_dir: str, arrays: dict, suffix: str = "", budget: int = 64 << 20):
+    """Writes `arrays` (name -> float array with one entry per request of a step) as out_dir/<name><suffix>.npy.  If
+    they come to more than `budget` bytes, the same fixed, seeded sample of requests is kept from every array and the
+    sampled request positions are written as `index`."""
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a.itemsize for a in arrays.values())
+    if n * row_bytes > budget:
+        keep = budget // (row_bytes + 8)
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}{suffix}.npy"), a)
 
 
 def _mix64(x):
@@ -722,7 +740,13 @@ def main():
     ap.add_argument("--leg", default="", choices=["", "rls", "ns_metrics"],
                     help="(internal) run ONE extra leg in this process and print its JSON: the parent run isolates the legs that "
                          "launch entry points beside the headline path in a child process")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (verdicts as float32 "
+                         "limited.npy; with one GPU also the first limited limit id as float64 first_limited.npy, "
+                         "0xFFFFFFFF = none) into DIR; with N GPUs every rank writes limited.rank<r>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs (--impl ours)")
     if args.leg:
         run_leg_child(args.leg)
         return
@@ -950,6 +974,13 @@ def main():
     if args.trace:
         with open(f"{args.trace}.rank{rank}.json", "w") as f:
             json.dump(eng.trace_dump(), f)
+    if args.dump_outputs:
+        # read before pass B: when the stream pool is cycled, pass B reuses these output slots
+        last = W + K - 1
+        outs = {"limited": out_lim[last].cpu().numpy().astype(np.float32)}
+        if world == 1:  # the sharded paths do not return the first limited limit
+            outs["first_limited"] = out_first[last].cpu().numpy().view(np.uint32).astype(np.float64)
+        dump_outputs(args.dump_outputs, outs, "" if world == 1 else f".rank{rank}", (64 << 20) // world)
     if args.device_pass_only:
         return
     value = world * batch * K / (ms_a * 1e-3)
