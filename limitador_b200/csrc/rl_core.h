@@ -32,6 +32,7 @@ enum : uint32_t {
     RL_DEV_TOO_MANY_COUNTERS = 4,  // > RL_MAX_CTRS_PER_REQ counters in one request
     RL_DEV_GROUP_SPLIT = 5,        // one request touches > RL_MAX_CELLS cells of one row (cannot happen)
     RL_DEV_EXCHANGE = 6,           // peer exchange: a rank's step flag did not arrive in time / a block fill is out of range
+    RL_DEV_CLOCK = 7,              // now_us == 0: an entry stored at expiry 0 would read as absent (RlRow)
 };
 
 // Per-(row group, cell) limit parameters.  max_value lives here and never in the row,

@@ -344,6 +344,8 @@ int check_device_error(rl_engine* e) {
             return fail(e, RL_FATAL, "key_hi bits 32..55 must be zero (counter identity is a 96-bit digest)");
         case RL_DEV_TOO_MANY_COUNTERS:
             return fail(e, RL_FATAL, "a request has more than %d counters", RL_MAX_CTRS_PER_REQ);
+        case RL_DEV_CLOCK:
+            return fail(e, RL_FATAL, "now_us must be >= 1");
         case RL_DEV_EXCHANGE: {
             const uint32_t d = e->h_misc[7];
             RL_CUDA(e, cudaMemsetAsync(e->d_misc.p + 7, 0, sizeof(uint32_t), e->stream));
@@ -1523,6 +1525,10 @@ static int stage_csr(rl_engine* e, uint64_t n, const uint32_t* off, const rl_cou
         d.total = last;
     } else {
         d.total = off[n];
+        for (uint64_t i = 0; i < n; i++)
+            if (now[i] == 0)
+                return fail(e, RL_FATAL, "now_us[%llu] must be >= 1 — the call was refused before the table was touched",
+                            (unsigned long long)i);
         if (d.total > e->max_counters)
             return fail(e, RL_FATAL, "batch has %llu counters > max_counters=%u", (unsigned long long)d.total, e->max_counters);
         RL_CUDA(e, e->d_in_off.reserve(e->max_batch + 1));
@@ -1569,7 +1575,7 @@ int rl_check_and_update_batch(rl_engine* e, uint64_t n, const uint32_t* ctr_off,
     o.off = c.off;
     RlDev D = make_dev(e);
     RlResolveOut O{e->d_acc.p, nullptr, nullptr, o.limited, o.first};
-    k_resolve_csr<<<ceil_div(n, 128), 128, 0, e->stream>>>(D, (uint32_t)n, c.off, c.ctrs, O, 1);
+    k_resolve_csr<<<ceil_div(n, 128), 128, 0, e->stream>>>(D, (uint32_t)n, c.off, c.ctrs, c.now, O, 1);
     RL_LAUNCH_CHECK(e);
     if ((r = check_resolve_error(e))) return r;
     if (c.total) {
@@ -1601,7 +1607,7 @@ int rl_update_batch(rl_engine* e, uint64_t n, const uint32_t* ctr_off, const rl_
     Outs o;
     RlDev D = make_dev(e);
     RlResolveOut O{e->d_acc.p, nullptr, nullptr, nullptr, nullptr};
-    k_resolve_csr<<<ceil_div(n, 128), 128, 0, e->stream>>>(D, (uint32_t)n, c.off, c.ctrs, O, 0);
+    k_resolve_csr<<<ceil_div(n, 128), 128, 0, e->stream>>>(D, (uint32_t)n, c.off, c.ctrs, c.now, O, 0);
     RL_LAUNCH_CHECK(e);
     if ((r = check_resolve_error(e))) return r;
     if ((r = run_acc_pipeline(e, (uint32_t)c.total, (uint32_t)n, c.delta, c.now, 2, 0, o))) return r;

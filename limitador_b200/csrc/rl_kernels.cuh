@@ -307,13 +307,18 @@ struct RecordSrc {
         if (ns_id >= D.ns_cap) return 0;
         const RlNsDev ns = D.ns[ns_id];
         if (ns.mode != 1) return 0;
+        if (!compact) {
+            const ulonglong2 w1 = rl_ld_stream(reinterpret_cast<const ulonglong2*>(r) + 1);  // key_hi, now_us
+            if (w1.y == 0) {  // 1 <= now_us: a cell stored at expiry 0 would read as absent
+                rl_set_err(D, RL_DEV_CLOCK);
+                return -1;
+            }
+            key_hi = w1.x & RL_RECORD_KEY_HI_MASK;
+        }
         if (ns.qualified_row) {
-            if (!compact) {
-                key_hi = __ldcs(reinterpret_cast<const unsigned long long*>(r) + 2) & RL_RECORD_KEY_HI_MASK;
-                if (key_hi >> 32) {
-                    rl_set_err(D, RL_DEV_KEY_RANGE);
-                    return -1;
-                }
+            if (!compact && (key_hi >> 32)) {
+                rl_set_err(D, RL_DEV_KEY_RANGE);
+                return -1;
             }
             key_lo = w0.y;
             hdr_hi = ((uint64_t)ns.group << 32) | key_hi;
@@ -1761,7 +1766,8 @@ struct RlResolveOut {
 };
 
 __global__ void k_resolve_csr(RlDev D, uint32_t n, const uint32_t* __restrict__ off,
-                              const rl_counter* __restrict__ ctrs, RlResolveOut O, int write_defaults) {
+                              const rl_counter* __restrict__ ctrs, const uint64_t* __restrict__ now, RlResolveOut O,
+                              int write_defaults) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const uint32_t o0 = off[i], m = off[i + 1] - o0;
@@ -1781,7 +1787,7 @@ __global__ void k_resolve_csr(RlDev D, uint32_t n, const uint32_t* __restrict__ 
         return r;
     };
     RlAccess tmp[RL_MAX_CTRS_PER_REQ];
-    const int nacc = rl_resolve_request(i, m, get, D.limits, D.limits_cap, true, tmp);
+    const int nacc = now[i] == 0 ? -(int)RL_DEV_CLOCK : rl_resolve_request(i, m, get, D.limits, D.limits_cap, true, tmp);
     if (nacc < 0) {
         rl_set_err(D, (uint32_t)(-nacc));
         for (uint32_t x = 0; x < m && x < RL_MAX_CTRS_PER_REQ; x++) {
@@ -1847,7 +1853,8 @@ __global__ void k_resolve_records(RlDev D, uint32_t n, const rl_record* __restri
         return r;
     };
     RlAccess tmp[RL_MAX_CTRS_PER_REQ];
-    const int nacc = rl_resolve_request(i, m, get, D.limits, D.limits_cap, true, tmp);
+    const int nacc =
+        rec.now_us == 0 ? -(int)RL_DEV_CLOCK : rl_resolve_request(i, m, get, D.limits, D.limits_cap, true, tmp);
     if (nacc < 0) {
         rl_set_err(D, (uint32_t)(-nacc));
         for (uint32_t x = 0; x < stride; x++) O.acc[o0 + x] = z;
